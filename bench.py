@@ -19,6 +19,9 @@ norm).  Speculative re-solves the GPU path performs on top of that are NOT count
 `--impl reference` times the reference's CPU algorithm (the oracle port: /root/reference is pure Python + two
 absent third-party solvers and cannot travel to the GPU box) on all host threads, on a bounded sample.
 
+`--dump-outputs DIR` writes what the timed path returned in its last step, the final labels, as DIR/labels.npy (float64).
+The workload and the permutations are seeded, so two builds run with the same arguments can be compared label for label.
+
 N > 1 (torchrun): queries are sharded over ranks, the per-round label exchange is an NCCL all-reduce; the workload is
 the same total problem (strong scaling).
 """
@@ -54,6 +57,8 @@ def parse_args():
     ap.add_argument("--no-qp-isolated", action="store_true")
     ap.add_argument("--scale-workloads", default="100k,1m",
                     help="other BASELINE workloads timed briefly at this N (stage ms in `scale_workloads`); '' to skip")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the labels of the last timed step as DIR/labels.npy (float64) to compare two builds")
     return ap.parse_args()
 
 
@@ -252,9 +257,11 @@ def run_reference(args):
     per_step_seconds = max(2.0, min(args.cpu_seconds, 150.0 / max(args.steps + args.warmup, 1)))
     vals, steps_used = [], 0
     for i in range(args.warmup + args.steps):
-        v, steps_used, dt = cpu_sample(X, bins, cfg, per_step_seconds, threads)
+        v, steps_used, dt, labels, _ = cpu_sample(X, bins, cfg, per_step_seconds, threads, return_labels=True)
         if i >= args.warmup:
             vals.append((v, dt))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, labels=labels)
     qps = float(np.mean([v for v, _ in vals]))
     ms = float(np.mean([dt for _, dt in vals]) * 1e3)
     sample = (f"first {steps_used} sequential steps of iteration 1 ({steps_used * cfg['C']} QPs) of the {args.workload} workload, "
@@ -484,6 +491,8 @@ def run_b200(args):
             scale[name] = {"error": repr(e)[:300]}
 
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, labels=labels_v)
         line = report(args, cfg, X, bins, U, world, elapsed_ms, elapsed_ms_b, total_iters, tmA, tm, fp64_peak, l2_gbs, clocks, value,
                       qps_ref_total, e2e_value, e2e_s, e2e_iters, same, e2e_pageable, scale, lab1, labels_v, R.perms, qp_iso, torch)
         _emit(line)
@@ -716,6 +725,24 @@ def report(args, cfg, X, bins, U, world, elapsed_ms, elapsed_ms_b, total_iters, 
         "peaks": {"fp64_tflops": fp64_peak, "l2_cap_gbs": l2_cap_gbs, "l2_gather_microbench_gbs": l2_gbs, "hbm_gbs": hbm_peak, "tf32_tflops": tf32_peak, "l2_bytes": l2_bytes},
         "clocks": clocks,
     }
+
+
+DUMP_MAX_ELEMENTS = 3_000_000  # per dump: values and their positions, 8 bytes each, stay below 64 MB
+
+
+def dump_outputs(out_dir, **arrays):
+    """Writes each array as out_dir/<name>.npy in float64 (exact for labels).  An array longer than its share of
+    DUMP_MAX_ELEMENTS is replaced by a fixed, seeded sample of its elements in position order; the positions go to
+    out_dir/<name>_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_MAX_ELEMENTS // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64).ravel()
+        if a.size > cap:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
+            a = a[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def _emit(line: dict):

@@ -94,7 +94,7 @@ def test_install_on_the_real_reference_module_through_the_ini_route(G, features_
     from oracle import ref_shim
 
     if not ref_shim.available():
-        pytest.skip("/root/reference is not mounted here (GPU box)")
+        pytest.skip(f"no reference project tree at {ref_shim.REFERENCE_ROOT} (CHB_REFERENCE_ROOT)")
     mod = ref_shim.load_cli_clustering()
     original = mod.perform_clustering
     seen = []
