@@ -24,8 +24,8 @@ EXPORTED_SYMBOLS = [
     "chb_set_labels", "chb_set_params", "chb_build_distance_matrix", "chb_get_distance_rows", "chb_knn_per_bin",
     "chb_hull_distance_batch", "chb_fit_iteration", "chb_fit", "chb_get_labels", "chb_iteration_begin", "chb_iteration_begin_dev", "chb_iteration_prefetch",
     "chb_round_run", "chb_round_commit", "chb_round_commit_end", "chb_iteration_end", "chb_set_window", "chb_get_window",
-    "chb_measure_fp64_tflops", "chb_measure_l2_gbs", "chb_guess_export", "chb_guess_import", "chb_set_distance_mode", "chb_set_gram_engine", "chb_get_candidate_rows", "chb_get_pair_cache",
-    "chb_get_fused_candidates", "chb_set_features_async", "chb_set_features_colmajor", "chb_set_features_merged", "chb_get_features",
+    "chb_measure_fp64_tflops", "chb_measure_l2_gbs", "chb_guess_export", "chb_guess_import", "chb_set_distance_mode", "chb_get_distance_path", "chb_set_gram_engine", "chb_get_candidate_rows", "chb_get_pair_cache",
+    "chb_get_fused_candidates", "chb_get_row_bounds", "chb_set_features_async", "chb_set_features_colmajor", "chb_set_features_merged", "chb_get_features",
 ]
 
 
@@ -114,6 +114,8 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
     L.chb_measure_l2_gbs.argtypes = [_vp, ctypes.POINTER(_dbl)]
     L.chb_guess_export.argtypes = [_vp, _vp, ctypes.POINTER(_i32)]
     L.chb_guess_import.argtypes = [_vp, _vp]
+    L.chb_get_distance_path.argtypes = [_vp, ctypes.POINTER(_i32)]
+    L.chb_get_row_bounds.argtypes = [_vp, _i64, _i64, _vp, _vp, _vp]
     for name in EXPORTED_SYMBOLS:
         fn = getattr(L, name)
         if name not in ("chb_last_error", "chb_get_window"):
@@ -274,6 +276,13 @@ class Context:
         """1 = FP32 candidate filter + exact FP64 re-rank (default), 0 = exact FP64 rows."""
         self._check(self._lib.chb_set_distance_mode(self._h, int(mode)))
 
+    def distance_path(self) -> int:
+        """The distance mode the rounds will run for the current features, labels, parameters and mode: 2 = fused path,
+        1 = FP32 candidate filter, 0 = exact rows (mode 2 falls back to 1 where the fused path does not serve)."""
+        out = _i32(0)
+        self._check(self._lib.chb_get_distance_path(self._h, ctypes.byref(out)))
+        return int(out.value)
+
     def set_gram_engine(self, engine: int):
         """1 = tcgen05 TF32x3 tensor-core Gram (default), 0 = FFMA Gram."""
         self._check(self._lib.chb_set_gram_engine(self._h, int(engine)))
@@ -296,6 +305,14 @@ class Context:
         key = key.reshape(-1)[:m].reshape(nslots, self.C, 2 * kr.value)
         idx = idx.reshape(-1)[:m].reshape(nslots, self.C, 2 * kr.value)
         return key, idx, np.ascontiguousarray(slack.T)
+
+    def get_row_bounds(self, slot0: int, nslots: int):
+        """Test aid (fused path): (guessed bin, ub, ubk2) of each owned slot -- the bin-pruning bounds."""
+        guess = np.empty(nslots, dtype=np.int32)
+        ub = np.empty(nslots, dtype=np.float32)
+        ubk2 = np.empty(nslots, dtype=np.float32)
+        self._check(self._lib.chb_get_row_bounds(self._h, slot0, nslots, _ptr(guess), _ptr(ub), _ptr(ubk2)))
+        return guess, ub, ubk2
 
     def get_pair_cache(self, slot0: int, nslots: int):
         idx = np.empty((nslots, self.C, self.k), dtype=np.int32)

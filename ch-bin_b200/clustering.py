@@ -395,7 +395,8 @@ def fit_cluster(
         ctx.set_distance_mode(int(distance_mode))
         ctx.set_gram_engine(int(gram_engine))
         spec_perm = spec_state = None  # a permutation drawn ahead of the iteration that will use it
-        on_device = world > 1 and dist_mod.get_backend() == "nccl" and int(distance_mode) == 2 and np.shape(samples)[1] <= 160
+        # the permutation stays on the device when the library's fused path serves the stage (chb_get_distance_path)
+        on_device = world > 1 and dist_mod.get_backend() == "nccl" and ctx.distance_path() == 2
         if max_iterations > 0:  # iteration 1 always executes: its permutation is drawn while the features are still in flight
             if world > 1:
                 with engine.stream_context():

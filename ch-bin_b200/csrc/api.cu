@@ -360,7 +360,7 @@ int ensure_caches(chb_ctx *c)
     if (c->cache_nown == nown && c->cache_C == c->C && c->cache_k == c->k && c->knn_idx) return CHB_OK;
     CHB_TRY(dev_reserve(c, &c->knn_idx, &c->cap_knn, nown * c->C * c->k));
     // exact distances of the cached lists: only the matrix-backed modes (knn.cu) keep them
-    if (!(c->dist_mode == 2 && c->filter_ok && chb_fused_supported(c)))
+    if (!chb_use_fused(c))
         CHB_TRY(dev_reserve(c, &c->knn_dist, &c->cap_knn_dist, nown * c->C * c->k));
     if (c->cap_pairs < nown * c->C) {
         CHB_TRY(dev_alloc(c, &c->knn_cnt, nown * c->C));
@@ -414,6 +414,27 @@ int sync_stream(chb_ctx *c)
 }
 
 } // namespace
+
+// Which path serves distance mode 2 -- decided here and nowhere else.  d <= 160: the fused kernel with the resident query
+// operand.  161 <= d <= 1024: the fused kernel with the streamed query operand once the STAGE has at least
+// WIDE_FUSED_MIN_PAIRS (query, point) pairs, U x n, else mode 1.  The pair count is the stage's, not the owned slice's, and
+// it is latched by chb_set_labels, so that every rank of a sharded stage -- and every call within one stage -- takes the
+// same path.  WIDE_FUSED_MIN_PAIRS is a compatibility floor, not a measured crossover: on a B200 at d = 200 the fused path
+// was faster at every size measured, down to 72 k pairs (DESIGN.md section 8, tools/wide_features.py); the floor keeps the
+// tiniest wide stages (< 250 k pairs, e.g. 500 contigs) on the mode-1 path they took before the streamed kernel existed.
+// CHB_WIDE_FUSED_MIN_PAIRS overrides it (read at chb_set_labels).  Otherwise (d > 1024, k > 32, features outside the FP32
+// filter's range) mode 1 or 0 serves.
+constexpr int64_t WIDE_FUSED_MIN_PAIRS = 250000;
+static int64_t wide_fused_min_pairs()
+{
+    const char *e = getenv("CHB_WIDE_FUSED_MIN_PAIRS");
+    return e ? (int64_t)atoll(e) : WIDE_FUSED_MIN_PAIRS;
+}
+bool chb_use_fused(const chb_ctx *c)
+{
+    if (!(c->dist_mode == 2 && c->filter_ok && chb_fused_supported(c))) return false;
+    return c->d <= CHB_FUSED_RESIDENT_DMAX || c->wide_fused_size_ok;
+}
 
 // =========================================================================================================
 extern "C" {
@@ -537,7 +558,7 @@ int chb_enable_timers(chb_ctx *c, int enable)
 }
 
 static inline bool use_filter(const chb_ctx *c) { return c->dist_mode >= 1 && c->filter_ok; }
-static inline bool use_fused(const chb_ctx *c) { return c->dist_mode == 2 && c->filter_ok && chb_fused_supported(c); }
+static inline bool use_fused(const chb_ctx *c) { return chb_use_fused(c); }
 
 // FP32 candidate rows for `nrows` query points (device list rows_dev), through the selected Gram engine
 static int candidate_rows(chb_ctx *c, const int32_t *rows_dev, int64_t nrows, float *out, int64_t ldo)
@@ -827,6 +848,13 @@ int chb_set_distance_mode(chb_ctx *c, int mode)
     return CHB_OK;
 }
 
+int chb_get_distance_path(chb_ctx *c, int32_t *mode_out)
+{
+    CHB_CHECK(c, c && mode_out, CHB_EINVAL, "NULL argument");
+    *mode_out = use_fused(c) ? 2 : (use_filter(c) ? 1 : 0);
+    return CHB_OK;
+}
+
 int chb_set_features(chb_ctx *c, const double *x, int64_t n, int32_t d)
 {
     return set_features_common(c, x, n, d, cudaMemcpyHostToDevice);
@@ -939,6 +967,7 @@ int chb_set_labels(chb_ctx *c, const int64_t *bins, int64_t n, int32_t C, int64_
     c->U = U;
     c->u0 = slot_begin;
     c->u1 = slot_end;
+    c->wide_fused_size_ok = U * n >= wide_fused_min_pairs(); // the stage's pair count: the same on every rank
     if (c->cap_n < n) {
         CHB_TRY(dev_alloc(c, &c->old_label, n));
         CHB_TRY(dev_alloc(c, &c->tent_pt, n));
@@ -1220,7 +1249,7 @@ int chb_iteration_prefetch(chb_ctx *c, const int64_t *perm, int64_t U)
 int chb_iteration_begin_dev(chb_ctx *c, const int64_t *perm_dev, int64_t U)
 {
     CHB_CHECK(c, c, CHB_EINVAL, "ctx is NULL");
-    CHB_CHECK(c, use_fused(c) || U == 0, CHB_EINVAL, "chb_iteration_begin_dev needs distance mode 2 (d <= 160); pass a host permutation otherwise");
+    CHB_CHECK(c, use_fused(c) || U == 0, CHB_EINVAL, "chb_iteration_begin_dev needs the fused path of distance mode 2 (chb_get_distance_path); pass a host permutation otherwise");
     return iteration_begin_common(c, perm_dev, U, true);
 }
 

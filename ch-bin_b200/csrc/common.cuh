@@ -55,6 +55,7 @@ struct chb_ctx {
     bool bsplit_ready = false;
     bool filter_ok = true; // feature magnitudes inside the FP32 filter's validated range
     bool nmax_pending = false; // the read-back deciding filter_ok is still in flight (chb_set_features_async)
+    bool wide_fused_size_ok = false; // 161 <= d <= 1024: the stage is large enough for the fused path (chb_set_labels)
 
     // ---- labels / slots
     int32_t C = 0;
@@ -300,7 +301,9 @@ int chb_launch_gram_tc(chb_ctx *ctx, const float *a_split, const float *b_split,
                        int64_t nrows, float *out_dev, int64_t ldo);
 
 // fused.cu : distance mode 2, Gram + per-bin selection in one tcgen05 kernel, then exact re-rank
-bool chb_fused_supported(const chb_ctx *c);
+constexpr int CHB_FUSED_RESIDENT_DMAX = 160; // widest d whose query operand stays resident in the fused kernel
+bool chb_fused_supported(const chb_ctx *c); // the kernels can serve this d and k
+bool chb_use_fused(const chb_ctx *c);       // api.cu: the rounds of this context run the fused path
 int chb_round_fused(chb_ctx *c);
 int chb_fused_setup(chb_ctx *c);  // allocations + once-per-label-set operands (idempotent)
 int chb_fused_grow_redo_list(chb_ctx *c); // exact-redo list to its worst-case size (every (row, bin) pair)

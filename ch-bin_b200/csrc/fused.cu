@@ -34,6 +34,7 @@
 #include <cuda.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdlib>
 
 #include "common.cuh"
@@ -48,11 +49,19 @@ constexpr int EPI_THREADS = 256;
 constexpr uint32_t TMEM_COLS = 256; // two 128-column accumulator buffers
 constexpr int MAX_BOX = 10;         // resident query operand: at most 10 boxes = 160 KB  (d <= 160)
 constexpr int SMEM_LIMIT = 232448;  // 227 KB opt-in shared memory per CTA
+constexpr int DMAX_F = CHB_FUSED_RESIDENT_DMAX; // resident query operand (d <= 160)
+constexpr int DMAX_W = 1024;        // streamed query operand (161 <= d <= 1024)
+constexpr int NKT_STREAMED = -1;    // gram_select_kernel's NKT for the streamed query operand
+constexpr int WIDE_STAGE_BOXES = 4; // streamed ring stage: {query hi, query lo, column hi, column lo} of one 32-feature block
 
-// Operand layout (queries and columns alike): row = [hi(dp8) | lo(dp8) | 0...] floats, dp8 = d rounded up to 8, padded to
-// nbox boxes of 32 floats.  hi/lo are the TF32 halves of the centred FP32 feature (gram_tc.cu).  The contraction
+// Operand layout (queries and columns alike), d <= 160: row = [hi(dp8) | lo(dp8) | 0...] floats, dp8 = d rounded up to 8,
+// padded to nbox boxes of 32 floats.  hi/lo are the TF32 halves of the centred FP32 feature (gram_tc.cu).  The contraction
 // hi.hi + hi.lo + lo.hi is issued as UMMA K=8 steps that pair step i of the RESIDENT query operand with step j of the
 // streamed column operand, so the query operand is read from L2 once per row block instead of once per tile.
+// d > 160: the query operand of a 128-row block no longer fits shared memory beside a ring.  Each half is padded to whole
+// boxes instead, row = [hi(dp32) | lo(dp32)], so that box b holds the hi parts of features 32b .. 32b + 31 and box H + b
+// (H = dp32 / 32) their lo parts; a ring stage carries the query AND column boxes of one 32-feature block and feeds
+// 4 K-steps x 3 products.  The operand builders take the half width as their `dp8` argument and zero-fill past d.
 constexpr int NC = 16; // per-thread candidate stack depth
 struct SmemTail {
     // candidates that passed the screen wait here (thread-private stacks, [slot][thread]; their columns are remembered in
@@ -319,8 +328,6 @@ __global__ void centre_finish_kernel(double *__restrict__ mc, const int32_t *__r
     if (threadIdx.x == 0) mc2[c] = red[0];
 }
 
-constexpr int DMAX_F = 160; // fused mode: d <= 160
-
 // |a_u - m_c|^2 for every query slot u and every bin c, once per label set: an FP64 GEMM (U x C x d) on the FP64 tensor cores
 // (mma.sync m8n8k4.f64 -> DMMA.8x8x4): 128 x 64 tiles per CTA, 8 warps of 32 x 32 (4 x 4 MMA tiles, 16 DMMA per 8 shared-memory
 // reads), 16 features per shared-memory stage, the next stage's global loads in flight behind the arithmetic.
@@ -563,8 +570,10 @@ __global__ void seed_transpose_kernel(const float *__restrict__ Xf, int32_t ldf,
 // contracts as well, and inflated rigorously: with D = x_q - x_s and D~ = a_q - a_s (exact difference of the stored floats),
 //   | D~ - D |_2 <= 2^-24 (|x_q - mu| + |x_s - mu|)            (one rounding per stored coordinate)
 //   S~ = fl32 sum of fl32(a_q,t - a_s,t)^2  >=  |D~|^2 (1 - (d + 3) 2^-24)   (all terms non-negative)
-// hence  |D| <= sqrt(S~) (1 + 1e-5) + 6e-8 (|a_q| + max_i |a_i|)  for d <= 160, every operation rounded upwards.  The pruning test
-// (threshold_kernel) keeps margins a hundred times wider than what this adds.
+// and 1 / sqrt(1 - x) <= 1 + x for 0 <= x <= 1/2, hence
+//   |D| <= sqrt(S~) f + 6e-8 (|a_q| + max_i |a_i|),   f = max(1 + 1e-5, 1 + (d + 3) 2^-24)   (ub_inflation)
+// every operation rounded upwards; f = 1 + 1e-5 up to d = 164, 1 + 6.1e-5 at d = 1024.  The pruning test (threshold_kernel)
+// keeps margins a hundred times wider than what this adds.
 //
 // Rows come grouped by guessed bin (row_end[c] = end of bin c's group), so a CTA takes 64 rows of ONE bin against that bin's
 // seeds: a register-tiled squared-distance "GEMM" -- 4 rows x 4 seeds per thread, operands staged through shared memory in
@@ -572,15 +581,21 @@ __global__ void seed_transpose_kernel(const float *__restrict__ Xf, int32_t ldf,
 // memory, up to RU_MAXSEED seeds per bin; beyond that only the minimum, ubk2 = +inf).
 constexpr int RU_ROWS = 64, RU_SEEDS = 32, RU_TK = 32, RU_THREADS = 128, RU_MAXSEED = 128;
 constexpr int RU_QP = RU_ROWS + 4, RU_DP = RU_MAXSEED + 1;
-__device__ __forceinline__ float ru_bound(float s2, float scale)
+inline float ub_inflation(int d)
 {
-    return __fadd_ru(__fmul_ru(__fsqrt_ru(s2), 1.00001f), __fmul_ru(6e-8f, scale));
+    const double f = 1.0 + (double)(d + 3) * 5.9604644775390625e-08;
+    const float fr = (float)f; // round to nearest: step up once if that went below
+    return std::max(1.00001f, (double)fr >= f ? fr : std::nextafter(fr, 2.f));
+}
+__device__ __forceinline__ float ru_bound(float s2, float scale, float inflate)
+{
+    return __fadd_ru(__fmul_ru(__fsqrt_ru(s2), inflate), __fmul_ru(6e-8f, scale));
 }
 __global__ void __launch_bounds__(RU_THREADS) row_ub_kernel(const int32_t *__restrict__ row_pt, int64_t nown, const float *__restrict__ Xf,
                                                             int32_t ldf, int32_t d, int32_t C, int32_t k, const int32_t *__restrict__ seed_off,
                                                             const float *__restrict__ seedT, int64_t ns, const int32_t *__restrict__ row_end,
                                                             const float *__restrict__ sq_row, const unsigned int *__restrict__ nrm_max_bits,
-                                                            float *__restrict__ ub_out, float *__restrict__ ubk2_out)
+                                                            float inflate, float *__restrict__ ub_out, float *__restrict__ ubk2_out)
 {
     chb_pdl_wait();
     __shared__ float dist[RU_ROWS * RU_DP];                 // 33 KB
@@ -705,8 +720,8 @@ __global__ void __launch_bounds__(RU_THREADS) row_ub_kernel(const int32_t *__res
         }
         if (lane == 0) {
             const float scale = __fadd_ru(sq_row[r0 + rr], amax);
-            ub_out[r0 + rr] = mn2 < INFINITY ? ru_bound(mn2, scale) : INFINITY;
-            const float bk = kth < INFINITY ? ru_bound(kth, scale) : INFINITY;
+            ub_out[r0 + rr] = mn2 < INFINITY ? ru_bound(mn2, scale, inflate) : INFINITY;
+            const float bk = kth < INFINITY ? ru_bound(kth, scale, inflate) : INFINITY;
             ubk2_out[r0 + rr] = bk < INFINITY ? __fmul_ru(bk, bk) : INFINITY;
         }
     }
@@ -1034,7 +1049,9 @@ __global__ void __launch_bounds__(1024) pairs_plan_kernel(const int32_t *__restr
 // buffer; one warp per row.  threshold_kernel left every pair's index inside its bin in row_pid: id = pair_off[bin] + index
 // (lane j resolves the row's j-th surviving bin), the operand row is read once and written once per pair.  Padding ids
 // keep pair_row = -1 (round_reset_kernel); their operand rows are never initialised -- accumulator rows are independent
-// and the epilogue ignores rows without a query.
+// and the epilogue ignores rows without a query.  WIDE = false: rows of up to 96 float4 (d <= 160) stay in registers,
+// three per lane; WIDE = true (streamed layout, up to 512 float4): the row is read again (L1) for every copy.
+template <bool WIDE>
 __global__ void __launch_bounds__(256) pairs_fill_kernel(const int32_t *__restrict__ mode, const int32_t *__restrict__ row_nb,
                                                          const int32_t *__restrict__ row_bins, int64_t nown, int32_t C,
                                                          const int32_t *__restrict__ pair_off, int32_t *__restrict__ pair_row,
@@ -1049,10 +1066,12 @@ __global__ void __launch_bounds__(256) pairs_fill_kernel(const int32_t *__restri
     const int nb = row_nb[r];
     if (nb == 0) return;
     const float4 *src = reinterpret_cast<const float4 *>(a2 + r * Kp2);
-    const int nq = Kp2 / 4; // <= 96 float4 per row (d <= 160): three per lane
+    const int nq = Kp2 / 4;
     float4 v[3];
+    if constexpr (!WIDE) {
 #pragma unroll
-    for (int u = 0; u < 3; ++u) v[u] = (lane + 32 * u < nq) ? __ldg(src + lane + 32 * u) : make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int u = 0; u < 3; ++u) v[u] = (lane + 32 * u < nq) ? __ldg(src + lane + 32 * u) : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
     for (int jb = 0; jb < nb; jb += 32) {
         const int j = jb + lane;
         int id = -1;
@@ -1066,9 +1085,13 @@ __global__ void __launch_bounds__(256) pairs_fill_kernel(const int32_t *__restri
         for (int w = 0; w < cnt; ++w) {
             const int idw = __shfl_sync(CHB_FULL, id, w);
             float4 *dst = reinterpret_cast<float4 *>(ap + (int64_t)idw * Kp2);
+            if constexpr (WIDE) {
+                for (int u = lane; u < nq; u += 32) dst[u] = __ldg(src + u);
+            } else {
 #pragma unroll
-            for (int u = 0; u < 3; ++u)
-                if (lane + 32 * u < nq) dst[lane + 32 * u] = v[u];
+                for (int u = 0; u < 3; ++u)
+                    if (lane + 32 * u < nq) dst[lane + 32 * u] = v[u];
+            }
         }
     }
 }
@@ -1108,7 +1131,9 @@ struct TopList {
 
 // NKT > 0: the number of K=8 steps per operand half is known at compile time and a tile's MMA sequence is straight-line
 // code with immediate descriptor offsets (d = 137..160, the reference's 4-mer + coverage profiles); NKT = 0: any d, the
-// sequence is tabulated in shared memory once per CTA.
+// sequence is tabulated in shared memory once per CTA; NKT = NKT_STREAMED: d = 161..1024, the query operand streams through
+// the ring with the column operand (one stage per 32-feature block, see the layout note at the top).  Only the producer and
+// MMA warps differ between the variants; the selection epilogue is the same code.
 template <int KR, int NKT>
 __global__ void __launch_bounds__(FUSED_THREADS, 1)
 gram_select_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_ap,
@@ -1129,12 +1154,15 @@ gram_select_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_const
     // mode 1: item.x is a block of 128 compact (row, bin) pairs of bin item.y, operand rows in the compact buffer (map_ap),
     // pair_row[] names the query row of each; mode 0: item.x is a row block of the resident operand (map_a)
     const int mode = *mode_p;
-    // dynamic shared memory: [resident query operand: nbox boxes][column ring: nstage boxes][SmemTail]
+    // dynamic shared memory: [resident query operand: nbox boxes][column ring: nstage boxes][SmemTail]; streamed:
+    // [ring: nstage x 4 boxes][SmemTail]
+    constexpr bool STREAM = NKT == NKT_STREAMED;
+    constexpr uint32_t STAGE_BYTES = STREAM ? WIDE_STAGE_BOXES * TILE_BYTES : TILE_BYTES;
     extern __shared__ uint8_t smem_raw[];
     uint8_t *base = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint8_t *a_res = base;
-    uint8_t *ring = base + (size_t)nbox * TILE_BYTES;
-    SmemTail &S = *reinterpret_cast<SmemTail *>(ring + (size_t)nstage * TILE_BYTES);
+    uint8_t *ring = STREAM ? base : base + (size_t)nbox * TILE_BYTES;
+    SmemTail &S = *reinterpret_cast<SmemTail *>(ring + (size_t)nstage * STAGE_BYTES);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
     if (threadIdx.x == 0) {
@@ -1170,6 +1198,24 @@ gram_select_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_const
             int cur_rb = -1, na = 0; // row block whose operand is resident, number of operand loads so far
             for (int it = item_begin; it < item_end; ++it) {
                 const int4 item = items[it];
+                if constexpr (STREAM) {
+                    // per tile and 32-feature block b: query boxes b (hi), H + b (lo) and column boxes b, H + b in one stage
+                    const int H = nbox >> 1;
+                    const CUtensorMap *mq = mode ? &map_ap : &map_a;
+                    for (int t = item.z; t < item.z + item.w; ++t) {
+                        for (int b = 0; b < H; ++b) {
+                            uint8_t *st = ring + (size_t)s * STAGE_BYTES;
+                            mbar_wait(&S.empty_bar[s], ph ^ 1);
+                            mbar_expect_tx(&S.full_bar[s], STAGE_BYTES);
+                            tma_load_2d(st, mq, &S.full_bar[s], b * BK, item.x * BM);
+                            tma_load_2d(st + TILE_BYTES, mq, &S.full_bar[s], (H + b) * BK, item.x * BM);
+                            tma_load_2d(st + 2 * TILE_BYTES, &map_b, &S.full_bar[s], b * BK, t * BN);
+                            tma_load_2d(st + 3 * TILE_BYTES, &map_b, &S.full_bar[s], (H + b) * BK, t * BN);
+                            if (++s == nstage) { s = 0; ph ^= 1; }
+                        }
+                    }
+                    continue;
+                }
                 if (item.x != cur_rb) {
                     // the resident operand may be overwritten once every MMA of the previous row block has completed
                     mbar_wait(&S.a_empty_bar, (uint32_t)((na & 1) ^ 1));
@@ -1227,7 +1273,7 @@ gram_select_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_const
             int cur_rb = -1, na = 0;
             for (int it = item_begin; it < item_end; ++it) {
                 const int4 item = items[it];
-                if (item.x != cur_rb) {
+                if (!STREAM && item.x != cur_rb) {
                     // every MMA on the previous row block's operand has been issued: release it, then wait for the new one
                     if (cur_rb >= 0 && elect_one_sync()) umma_commit(&S.a_empty_bar);
                     mbar_wait(&S.a_full_bar, (uint32_t)(na & 1));
@@ -1242,7 +1288,31 @@ gram_select_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_const
                     mbar_wait(&S.tmem_empty_bar[buf], tph ^ 1); // epilogue has drained this accumulator buffer
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     const uint32_t tmem_d = tmem_base + (uint32_t)(buf * BN);
-                    if constexpr (NKT > 0) {
+                    if constexpr (STREAM) {
+                        // stage = [query hi | query lo | column hi | column lo] of one 32-feature block: 4 K-steps x
+                        // (hi.hi, lo.hi, hi.lo); zero pads past d contribute exact zeros
+                        const int H = nbox >> 1;
+                        for (int b = 0; b < H; ++b) {
+                            const uint32_t st_lo = ring_lo + (uint32_t)s * (STAGE_BYTES >> 4);
+                            mbar_wait(&S.full_bar[s], ph);
+                            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                            if (elect_one_sync()) {
+#pragma unroll
+                                for (int u = 0; u < BK / UMMA_K; ++u) {
+                                    const uint32_t ko = (uint32_t)((u * UMMA_K * 4) >> 4);
+                                    const uint64_t qhi = ((uint64_t)DESC_HI << 32) | (st_lo + ko);
+                                    const uint64_t qlo = ((uint64_t)DESC_HI << 32) | (st_lo + (TILE_BYTES >> 4) + ko);
+                                    const uint64_t chi = ((uint64_t)DESC_HI << 32) | (st_lo + 2 * (TILE_BYTES >> 4) + ko);
+                                    const uint64_t clo = ((uint64_t)DESC_HI << 32) | (st_lo + 3 * (TILE_BYTES >> 4) + ko);
+                                    umma_tf32(tmem_d, qhi, chi, idesc, (b | u) != 0);
+                                    umma_tf32(tmem_d, qlo, chi, idesc, 1u);
+                                    umma_tf32(tmem_d, qhi, clo, idesc, 1u);
+                                }
+                                umma_commit(&S.empty_bar[s]);
+                            }
+                            if (++s == nstage) { s = 0; ph ^= 1; }
+                        }
+                    } else if constexpr (NKT > 0) {
                         constexpr int NBOX = (2 * NKT + 3) / 4;
                         const uint32_t a_lo = ((a_addr & 0x3FFFFu) >> 4) | (1u << 16);
 #pragma unroll
@@ -2253,18 +2323,32 @@ int make_map(chb_ctx *ctx, CUtensorMap *map, float *base, int64_t nrows, int32_t
     return CHB_OK;
 }
 
+// dp8 = width of one operand half (d rounded up to 8, or to 32 when streamed), nk = its K=8 steps, nbox = 32-float boxes per
+// operand row, Kp2 = floats per operand row, nstage = ring stages (boxes, or 4-box stages when streamed)
 struct FusedGeom {
     int dp8, nk, nbox, Kp2, nstage;
+    bool stream;
     size_t smem;
 };
 FusedGeom fused_geom(int d)
 {
     FusedGeom g{};
+    const int fixed = 1024 + (int)sizeof(SmemTail);
+    g.stream = d > DMAX_F;
+    if (g.stream) {
+        g.dp8 = (d + BK - 1) & ~(BK - 1);
+        g.nk = g.dp8 / UMMA_K;
+        g.nbox = 2 * g.dp8 / BK;
+        g.Kp2 = g.nbox * BK;
+        const int stage = WIDE_STAGE_BOXES * (int)TILE_BYTES;
+        g.nstage = std::min(8, (SMEM_LIMIT - fixed) / stage);
+        g.smem = (size_t)fixed + (size_t)g.nstage * stage;
+        return g;
+    }
     g.dp8 = (d + 7) & ~7;
     g.nk = g.dp8 / UMMA_K;
     g.nbox = (2 * g.dp8 + BK - 1) / BK;
     g.Kp2 = g.nbox * BK;
-    const int fixed = 1024 + (int)sizeof(SmemTail);
     g.nstage = std::min(8, (SMEM_LIMIT - fixed - g.nbox * (int)TILE_BYTES) / (int)TILE_BYTES);
     g.smem = (size_t)fixed + (size_t)(g.nbox + std::max(g.nstage, 0)) * TILE_BYTES;
     return g;
@@ -2288,6 +2372,7 @@ int launch_fused(chb_ctx *c, const CUtensorMap &ma, const CUtensorMap &map, cons
 template <int KR>
 int dispatch_nk(chb_ctx *c, const CUtensorMap &ma, const CUtensorMap &map, const CUtensorMap &mb, int64_t nrows, const FusedGeom &g)
 {
+    if (g.stream) return launch_fused<KR, NKT_STREAMED>(c, ma, map, mb, nrows, g);
     const bool generic = getenv("CHB_FUSED_GENERIC") != nullptr; // test aid: force the tabulated MMA sequence
     if (!generic && g.nk == 18) return launch_fused<KR, 18>(c, ma, map, mb, nrows, g);
     if (!generic && g.nk == 19) return launch_fused<KR, 19>(c, ma, map, mb, nrows, g);
@@ -2321,13 +2406,15 @@ inline unsigned nblk(int64_t n, int t) { return (unsigned)((n + t - 1) / t); }
 
 } // namespace
 
-// the resident query operand (2 * dp8 floats per row) fits MAX_BOX boxes with at least 3 ring stages left; up to k = 15 the
-// k + 1 candidates the re-rank needs fit a 16-entry register half-list of the fused kernel, larger k uses pruning + exact
-// selection only (chb_round_fused)
+// d <= 160: the resident query operand (2 * dp8 floats per row) fits MAX_BOX boxes with at least 3 ring stages left;
+// 161 <= d <= 1024: the streamed kernel, 3 stages of 64 KB.  Up to k = 15 the k + 1 candidates the re-rank needs fit a
+// 16-entry register half-list of the fused kernel, larger k uses pruning + exact selection only (chb_round_fused).  Whether
+// a stage runs on this path is decided by chb_use_fused (api.cu) from the input size as well.
 bool chb_fused_supported(const chb_ctx *c)
 {
     const FusedGeom g = fused_geom(c->d);
-    return c->k <= XS_KEEP && g.nbox <= MAX_BOX && g.nstage >= 3;
+    if (c->k > XS_KEEP || c->d > DMAX_W) return false;
+    return g.nstage >= 3 && (g.stream || g.nbox <= MAX_BOX);
 }
 
 void chb_fused_free(chb_ctx *c)
@@ -2412,7 +2499,7 @@ extern "C" int chb_guess_export(chb_ctx *c, int32_t *guess_dev, int32_t *active)
     CHB_CHECK(c, c && guess_dev && active, CHB_EINVAL, "NULL argument");
     CHB_CHECK(c, c->labels_set && c->dist_ready, CHB_EINVAL, "guess_export: labels / distance structure not set up");
     *active = 0;
-    if (!(c->dist_mode == 2 && c->filter_ok && chb_fused_supported(c)) || c->U <= 0 || !c->guess_pending) return CHB_OK;
+    if (!chb_use_fused(c) || c->U <= 0 || !c->guess_pending) return CHB_OK;
     CHB_CUDA(c, cudaSetDevice(c->device));
     if (!c->guess_shared) { c->guess_shared = true; c->f_asplit_ready = false; }
     c->guess_imported = false;
@@ -2452,7 +2539,7 @@ int chb_fused_setup(chb_ctx *c)
     const FusedGeom g = fused_geom(c->d);
     const int64_t ncol_max = ((2 * n + (int64_t)BN * C + BN - 1) / BN) * BN;
 
-    CHB_CHECK(c, chb_fused_supported(c), CHB_EINVAL, "fused mode supports num_neighbors <= 32 and d <= 160");
+    CHB_CHECK(c, chb_fused_supported(c), CHB_EINVAL, "fused mode supports num_neighbors <= 32 and d <= 1024");
     if (c->f_cap_bins < C + 1) {
         int64_t z = 0;
         z = 0; if (reserve(c, &c->f_bin_cnt, &z, C + 1)) return CHB_ENOMEM;
@@ -2599,7 +2686,7 @@ int chb_fused_setup(chb_ctx *c)
             }
             row_ub_kernel<<<(unsigned)(nown / RU_ROWS + C + 2), RU_THREADS, 0, side>>>(
                 c->f_row_pt, nown, c->Xf, c->ldf, c->d, C, k, c->seed_off, c->f_seedT, n - c->U, c->f_rhist + C + 2, c->f_sq_row,
-                reinterpret_cast<const unsigned int *>(&c->counters[5]), c->f_ub, c->f_ubk2);
+                reinterpret_cast<const unsigned int *>(&c->counters[5]), ub_inflation(c->d), c->f_ub, c->f_ubk2);
             if (!no_side) {
                 CHB_CUDA(c, cudaEventRecord(c->ev_join, side));
                 c->side_join_pending = true;
@@ -2655,7 +2742,9 @@ int chb_round_fused(chb_ctx *c)
         c->side_join_pending = false;
     }
 
-    // ---- 2. error slack and admission thresholds per (query, bin), then the fused Gram + selection
+    // ---- 2. error slack and admission thresholds per (query, bin), then the fused Gram + selection.  eps_rel bounds the FP32
+    // accumulation of the 3d products whatever the order the MMAs issue them in (the bound of a sum of n terms holds for any
+    // summation tree); the streamed kernel's block-interleaved order and its zero pads past d (exact zeros) keep it.
     const double eps_rel = (double)(3 * c->d + 64) * 1.1920928955078125e-07;
     {
         const bool wide = nown * (int64_t)C >= (int64_t)1 << 24; // 16 M pairs and more: a stream over the pair table
@@ -2696,7 +2785,7 @@ int chb_round_fused(chb_ctx *c)
     CHB_PDL_LAUNCH(c, pairs_plan_kernel, 1, 1024, 0, bin_surv, c->f_seg_off, C, plan_cap, c->sm_count, pair_off,
                                                  c->f_pair_meta + 3 * (C + 2), c->f_items, c->f_cta_begin, &c->counters[7], c->f_mode,
                                                  c->f_cand_dense ? 1 : 0, c->f_skip, nrb);
-    CHB_PDL_LAUNCH(c, pairs_fill_kernel, nblk(nown * 32, 256), 256, 0, c->f_mode, c->f_row_nb, c->f_row_bins, nown, C, pair_off,
+    CHB_PDL_LAUNCH(c, g.stream ? pairs_fill_kernel<true> : pairs_fill_kernel<false>, nblk(nown * 32, 256), 256, 0, c->f_mode, c->f_row_nb, c->f_row_bins, nown, C, pair_off,
                    c->f_pair_row, c->f_row_pid, c->f_a2, g.Kp2, c->f_ap);
     CHB_CUDA(c, cudaGetLastError());
     c->tm.launches_other += 3;
@@ -2796,6 +2885,33 @@ extern "C" int chb_get_fused_candidates(chb_ctx *c, int64_t slot0, int64_t nslot
         for (int32_t b = 0; b < C; ++b) slack_out[(int64_t)b * nslots + sl] = srow[(size_t)b];
     }
     CHB_CUDA(c, cudaStreamSynchronize(c->stream));
+    return CHB_OK;
+}
+
+extern "C" int chb_get_row_bounds(chb_ctx *c, int64_t slot0, int64_t nslots, int32_t *guess_out, float *ub_out, float *ubk2_out)
+{
+    CHB_CHECK(c, c && guess_out && ub_out && ubk2_out, CHB_EINVAL, "NULL argument");
+    CHB_CHECK(c, c->f_ub && c->f_asplit_ready && slot0 >= c->u0 && nslots >= 0 && slot0 + nslots <= c->u1, CHB_EINVAL,
+              "slots not owned / the fused path has not set up this label set");
+    CHB_CUDA(c, cudaSetDevice(c->device));
+    if (c->side_join_pending) { // row_ub_kernel runs on the side stream
+        CHB_CUDA(c, cudaStreamWaitEvent(c->stream, c->ev_join, 0));
+        c->side_join_pending = false;
+    }
+    const int64_t nown = c->u1 - c->u0, s0 = slot0 - c->u0;
+    std::vector<int32_t> slot_row((size_t)std::max<int64_t>(nown, 1)), guess((size_t)std::max<int64_t>(nown, 1));
+    std::vector<float> ub((size_t)std::max<int64_t>(nown, 1)), ubk2((size_t)std::max<int64_t>(nown, 1));
+    CHB_CUDA(c, cudaMemcpyAsync(slot_row.data(), c->f_slot_row, sizeof(int32_t) * (size_t)nown, cudaMemcpyDeviceToHost, c->stream));
+    CHB_CUDA(c, cudaMemcpyAsync(guess.data(), c->f_row_guess, sizeof(int32_t) * (size_t)nown, cudaMemcpyDeviceToHost, c->stream));
+    CHB_CUDA(c, cudaMemcpyAsync(ub.data(), c->f_ub, sizeof(float) * (size_t)nown, cudaMemcpyDeviceToHost, c->stream));
+    CHB_CUDA(c, cudaMemcpyAsync(ubk2.data(), c->f_ubk2, sizeof(float) * (size_t)nown, cudaMemcpyDeviceToHost, c->stream));
+    CHB_CUDA(c, cudaStreamSynchronize(c->stream));
+    for (int64_t s = 0; s < nslots; ++s) {
+        const int64_t r = slot_row[(size_t)(s0 + s)];
+        guess_out[s] = guess[(size_t)r];
+        ub_out[s] = ub[(size_t)r];
+        ubk2_out[s] = ubk2[(size_t)r];
+    }
     return CHB_OK;
 }
 

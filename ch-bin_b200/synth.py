@@ -35,12 +35,14 @@ def make_contig_features(
     seed: int = 0,
     concentration: float = 4000.0,
     coverage_column: Optional[np.ndarray] = None,
+    kmer_dims: int = KMER_DIMS,
 ) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
-    """Returns (samples (n, 136+S) float64 C-contiguous, initial_bins (n,) int64 with -1 = unassigned,
-    true_genome (n,) int64)."""
+    """Returns (samples (n, kmer_dims+S) float64 C-contiguous, initial_bins (n,) int64 with -1 = unassigned,
+    true_genome (n,) int64).  kmer_dims: width of the k-mer profile, 136 canonical 4-mers by default; 512 gives
+    5-mer-like profiles."""
     rng = np.random.default_rng(seed)
     C, S = int(num_genomes), int(num_cov_samples)
-    centroids = rng.dirichlet(np.full(KMER_DIMS, 8.0), size=C)
+    centroids = rng.dirichlet(np.full(int(kmer_dims), 8.0), size=C)
     truth = rng.integers(0, C, size=n)
     # every genome needs at least n_seed members
     need = np.repeat(np.arange(C), n_seed)
@@ -48,7 +50,7 @@ def make_contig_features(
         raise ValueError("n too small for num_genomes * n_seed")
     truth[: len(need)] = need
     rng.shuffle(truth)
-    kmers = np.empty((n, KMER_DIMS))
+    kmers = np.empty((n, int(kmer_dims)))
     for c in range(C):
         idx = np.where(truth == c)[0]
         if len(idx):

@@ -145,14 +145,25 @@ int chb_set_params(chb_ctx *ctx, int32_t num_neighbors, int32_t metric);
  *   mode 2 (default): nothing is stored; every round the tensor cores regenerate error-bounded FP32 candidate values
  *           and the per-bin selection happens in the same kernel's epilogue (fused.cu); exact scipy-cdist values are
  *           evaluated only where the FP32 bound cannot decide.  Bins that provably cannot be a query's nearest hull are
- *           pruned first.  num_neighbors >= 14: pruning, then exact selection for the surviving pairs (no Gram kernel).
- *           Needs d <= 160, else mode 1 is used.
+ *           pruned first.  num_neighbors >= 25: pruning, then exact selection for the surviving pairs (no Gram kernel).
+ *           The library picks the kernel from the input: d <= 160 keeps a 128-row block's query operand resident in
+ *           shared memory; 161 <= d <= 1024 streams it through the TMA ring with the column operand, and runs only when
+ *           the stage has at least WIDE_FUSED_MIN_PAIRS = 250 000 (query, point) pairs, U x n over ALL query slots (the
+ *           same on every rank; latched by chb_set_labels, env CHB_WIDE_FUSED_MIN_PAIRS read there).  That value is a
+ *           compatibility floor that keeps tiny wide stages on mode 1, not a crossover: the fused path was faster at
+ *           every size measured.  Below it, and for d > 1024 or num_neighbors > 32, mode 1 serves
+ *           (chb_get_distance_path tells which).
  *   mode 1: the FP32 candidate matrix of the owned query rows is kept in HBM (InMemDistMatrix=yes) or recomputed per
  *           round (no) and scanned by knn.cu; exact values for candidates only.
  *   mode 0: every exact FP64 distance is formed (3 non-fusable FP64 ops per feature) and ranked directly.
  * In all modes the neighbour sets are bit-identical to ranking scipy's exact rows.  Call before
  * chb_build_distance_matrix. */
 int chb_set_distance_mode(chb_ctx *ctx, int mode);
+/* The distance mode the assignment rounds will run with the current features, labels, parameters and mode setting:
+ * 2 = the fused path, 1 = the FP32 candidate filter, 0 = exact rows.  Call after chb_set_labels / chb_set_params /
+ * chb_set_distance_mode.  After chb_set_features_async the features' magnitude check may still be in flight; it is then
+ * assumed to pass (it fails only for features near FP32 overflow or underflow). */
+int chb_get_distance_path(chb_ctx *ctx, int32_t *mode_out);
 /* Engine of the FP32 candidate values in distance mode 1: 1 (default) = tcgen05 tensor cores, TF32 with a 3-term
  * hi/lo split, TMA-fed, TMEM accumulators (gram_tc.cu); 0 = FFMA on the CUDA cores (approx.cu). */
 int chb_set_gram_engine(chb_ctx *ctx, int engine);
@@ -168,6 +179,10 @@ int chb_get_pair_cache(chb_ctx *ctx, int64_t slot0, int64_t nslots, int32_t *idx
  * key_out / idx_out: nslots * C * 32 entries must be available (only nslots * C * 2 * KR are written). */
 int chb_get_fused_candidates(chb_ctx *ctx, int64_t slot0, int64_t nslots, float *key_out, int32_t *idx_out, float *slack_out,
                              int32_t *kr_out);
+/* Test aid (fused path): the bin-pruning bounds of owned slots [slot0, slot0+nslots) for the current label set: the
+ * guessed bin (num_clusters = none), ub_out >= the distance to that bin's nearest seed contig, ubk2_out >= the squared
+ * distance to its k-th nearest seed (+inf when it has fewer than k or more than 128 seeds). */
+int chb_get_row_bounds(chb_ctx *ctx, int64_t slot0, int64_t nslots, int32_t *guess_out, float *ub_out, float *ubk2_out);
 /* create_in_mem_distance_matrix / create_distance_matrix (distance_matrix.py:12-44) for the owned query
  * rows.  materialise=1: rows are computed once (exact cdist recipe) and kept in HBM (InMemDistMatrix=yes,
  * cli/clustering.py:57-59); fails with CHB_ENOMEM if they do not fit.  materialise=0: nothing is stored,
