@@ -15,6 +15,7 @@ from . import build, capi, distance_cache, features, synth  # noqa: F401
 from .clustering import (  # noqa: F401
     B200_SOLVER,
     GpuEngine,
+    GroupEngine,
     TorchComm,
     draw_permutations,
     exchange_guess,
@@ -27,6 +28,6 @@ from .clustering import (  # noqa: F401
 )
 
 __all__ = [
-    "B200_SOLVER", "GpuEngine", "TorchComm", "draw_permutations", "exchange_guess", "fit_cluster", "install", "owned_slots", "perform_clustering",
+    "B200_SOLVER", "GpuEngine", "GroupEngine", "TorchComm", "draw_permutations", "exchange_guess", "fit_cluster", "install", "owned_slots", "perform_clustering",
     "run_iteration", "shutdown", "build", "capi", "distance_cache", "features", "synth",
 ]

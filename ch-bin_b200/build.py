@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB_PATH = os.path.join(HERE, "libchbin_b200.so")
-SOURCES = ["api.cu", "distance.cu", "knn.cu", "knn_exact.cu", "qp.cu", "qp_small.cu", "qp_mid.cu", "qp_lane.cu", "approx.cu", "gram_tc.cu", "fused.cu", "peak.cu"]
+SOURCES = ["api.cu", "distance.cu", "knn.cu", "knn_exact.cu", "qp.cu", "qp_small.cu", "qp_mid.cu", "qp_lane.cu", "approx.cu", "gram_tc.cu", "fused.cu", "peak.cu", "group.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17",

@@ -26,6 +26,7 @@ EXPORTED_SYMBOLS = [
     "chb_round_run", "chb_round_commit", "chb_round_commit_end", "chb_iteration_end", "chb_set_window", "chb_get_window",
     "chb_measure_fp64_tflops", "chb_measure_l2_gbs", "chb_guess_export", "chb_guess_import", "chb_set_distance_mode", "chb_get_distance_path", "chb_set_gram_engine", "chb_get_candidate_rows", "chb_get_pair_cache",
     "chb_get_fused_candidates", "chb_get_row_bounds", "chb_set_features_async", "chb_set_features_colmajor", "chb_set_features_merged", "chb_get_features",
+    "chb_group_create", "chb_group_destroy", "chb_group_buffer", "chb_group_all_max", "chb_group_replicate_features",
 ]
 
 
@@ -116,6 +117,11 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
     L.chb_guess_import.argtypes = [_vp, _vp]
     L.chb_get_distance_path.argtypes = [_vp, ctypes.POINTER(_i32)]
     L.chb_get_row_bounds.argtypes = [_vp, _i64, _i64, _vp, _vp, _vp]
+    L.chb_group_create.argtypes = [ctypes.POINTER(_vp), ctypes.POINTER(_vp), _i32]
+    L.chb_group_destroy.argtypes = [_vp]
+    L.chb_group_buffer.argtypes = [_vp, _i32, _i64, ctypes.POINTER(_vp)]
+    L.chb_group_all_max.argtypes = [_vp, _i64]
+    L.chb_group_replicate_features.argtypes = [_vp, _i32]
     for name in EXPORTED_SYMBOLS:
         fn = getattr(L, name)
         if name not in ("chb_last_error", "chb_get_window"):
@@ -435,3 +441,59 @@ class Context:
         nch = _i64(0)
         self._check(self._lib.chb_iteration_end(self._h, ctypes.byref(nch)))
         return int(nch.value)
+
+
+class Group:
+    """A device group (chb_group_*): N distinct contexts driven from this thread, exchanging int32 label windows on the
+    devices.  Holds its member Contexts; close the group before any of them."""
+
+    def __init__(self, members):
+        self._lib = load()
+        self.members = list(members)
+        if not self.members or any(getattr(m, "_h", None) is None for m in self.members):
+            raise ValueError("a device group needs at least one open context")
+        self._h = _vp()
+        arr = (_vp * len(self.members))(*[m._h for m in self.members])
+        self._check(self._lib.chb_group_create(ctypes.byref(self._h), arr, len(self.members)))
+        self._bufs = [None] * len(self.members)  # (device address, entries) per member
+
+    def _check(self, rc: int):
+        if rc == CHB_OK:
+            return
+        msg = self._lib.chb_last_error(None).decode()
+        if rc == CHB_EINVAL:
+            raise ValueError(msg)
+        if rc == CHB_ENOMEM:
+            raise MemoryError(msg)
+        raise RuntimeError(f"libchbin_b200 error {rc}: {msg}")
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.chb_group_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def buffer(self, m: int, count: int) -> int:
+        """Device address of member m's group buffer, grown to at least `count` int32 entries."""
+        cur = self._bufs[m]
+        if cur is None or cur[1] < count:
+            ptr = _vp()
+            self._check(self._lib.chb_group_buffer(self._h, int(m), int(count), ctypes.byref(ptr)))
+            cur = self._bufs[m] = (int(ptr.value), int(count))
+        return cur[0]
+
+    def all_max(self, count: int):
+        """Element-wise MAX of the members' buffers [0, count), into every member's buffer (enqueued only)."""
+        self._check(self._lib.chb_group_all_max(self._h, int(count)))
+
+    def replicate_features(self, root: int = 0):
+        """Member `root`'s feature matrix into every other member (enqueued; each receiver derives its own FP32 copy)."""
+        self._check(self._lib.chb_group_replicate_features(self._h, int(root)))
+        r = self.members[root]
+        for m in self.members:
+            m.n, m.d = r.n, r.d

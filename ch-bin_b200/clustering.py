@@ -10,7 +10,8 @@ Host-side mirror of the reference's clustering interface for the B200 path.
 All arithmetic of the hot path (distance rows, per-bin kNN, hull-distance QPs, ordered assignment) runs in
 libchbin_b200.so (hand-written sm_100a CUDA) behind the C-ABI of include/chbin_b200.h.  This module only owns
 what the reference keeps in Python: the permutation draws on numpy's global legacy RNG, the early-stop rule,
-logging, and -- when torch.distributed is initialised with more than one rank -- the per-round label exchange.
+logging, and -- when torch.distributed is initialised with more than one rank -- the per-round label exchange (a device
+group of fit_cluster(devices=...) exchanges the labels inside the library instead).
 There is no CPU fallback.
 """
 from __future__ import annotations
@@ -20,7 +21,7 @@ import os
 import shutil
 import time
 from pathlib import Path
-from typing import Optional, Tuple
+from typing import Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -37,20 +38,50 @@ _CTX_CACHE = {}
 # ... and one torch stream per device for the sharded path: torch's caching allocator keeps its pools per stream, so a fresh
 # stream per call would turn every torch.empty into a cudaMalloc (tens of milliseconds)
 _STREAM_CACHE = {}
+# Device groups of fit_cluster(devices=...), by device tuple, with their member contexts.  Member 0 is the device's ordinary
+# cached context; member i > 0 has a context of its own under (device, i), so that a device may appear more than once.
+_GROUP_CACHE = {}
 
 
-def _get_context(device: int, reuse: bool) -> "capi.Context":
+def _get_context(device: int, reuse: bool, member: int = 0) -> "capi.Context":
     if not reuse:
         return capi.Context(device)
-    ctx = _CTX_CACHE.get(device)
+    key = device if member == 0 else (device, member)
+    ctx = _CTX_CACHE.get(key)
     if ctx is None or getattr(ctx, "_h", None) is None:
         ctx = capi.Context(device)
-        _CTX_CACHE[device] = ctx
+        _CTX_CACHE[key] = ctx
     return ctx
 
 
+def _get_group(devices, members, reuse: bool) -> "capi.Group":
+    if not reuse:
+        return capi.Group(members)
+    key = tuple(devices)
+    g = _GROUP_CACHE.get(key)
+    if g is None or g._h is None or any(a is not b for a, b in zip(g.members, members)):
+        g = _GROUP_CACHE[key] = capi.Group(members)
+    return g
+
+
+def _drop(ctxs) -> None:
+    """Closes these contexts and every cached group that holds one of them (groups first: they refer to their members)."""
+    for key, g in list(_GROUP_CACHE.items()):
+        if any(m is c for m in g.members for c in ctxs):
+            g.close()
+            del _GROUP_CACHE[key]
+    for key, c in list(_CTX_CACHE.items()):
+        if any(c is x for x in ctxs):
+            del _CTX_CACHE[key]
+    for c in ctxs:
+        c.close()
+
+
 def shutdown() -> None:
-    """Destroys the cached per-device contexts (frees all device memory held by the library)."""
+    """Destroys the cached device groups and per-device contexts (frees all device memory held by the library)."""
+    for g in list(_GROUP_CACHE.values()):
+        g.close()
+    _GROUP_CACHE.clear()
     for ctx in list(_CTX_CACHE.values()):
         ctx.close()
     _CTX_CACHE.clear()
@@ -203,6 +234,64 @@ class _ContextEngine:
         return self.ctx.iteration_end()
 
 
+class GroupEngine:
+    """The round interface over a device group (capi.Group) in one process: every member runs the round of its owned slots
+    into its group buffer, then chb_group_all_max merges the windows by element-wise MAX on the devices -- what the NCCL
+    all-reduce does between ranks, without torch.  The members commit the same merged labels and must agree on the result."""
+
+    def __init__(self, group: "capi.Group", U: int):
+        self.group = group
+        self.members = group.members
+        self.bufs = [group.buffer(m, max(U, 1)) for m in range(len(self.members))]
+
+    def stream_context(self):
+        import contextlib
+
+        return contextlib.nullcontext()  # every member runs on its own stream
+
+    def window(self):
+        return self.members[0].get_window()
+
+    def iteration_begin(self, perm):
+        for m in self.members:
+            m.iteration_begin(perm)
+
+    def prefetch(self, perm):
+        for m in self.members:
+            m.iteration_prefetch(perm)
+
+    def round_run(self, lo, hi):
+        for m, b in zip(self.members, self.bufs):
+            m.round_run(lo, hi, b)
+        self.group.all_max(hi - lo)
+        return None
+
+    def _agree(self, results, what):
+        if any(r != results[0] for r in results):
+            raise RuntimeError(f"the members of the device group disagree on {what}: {results}")
+        return results[0]
+
+    def round_commit_end(self, lo, hi, tent):
+        return self._agree([m.round_commit_end(lo, hi, b) for m, b in zip(self.members, self.bufs)],
+                           "(first_changed, done, n_changed)")
+
+    def iteration_end(self):
+        return self._agree([m.iteration_end() for m in self.members], "n_changed")
+
+    def guess_export(self, U):
+        active = [m.guess_export(b) for m, b in zip(self.members, self.bufs)]
+        return U if self._agree(active, "the guess exchange") else None
+
+    def all_reduce_max(self, count):
+        """The guess exchange of exchange_guess: the same MAX over the members' buffers."""
+        self.group.all_max(count)
+        return count
+
+    def guess_import(self, g):
+        for m, b in zip(self.members, self.bufs):
+            m.guess_import(b)
+
+
 class TorchComm:
     """Label exchange between ranks: one all-reduce(MAX) of a window of int32 labels per round (un-owned
     positions hold INT32_MIN).  NCCL over NVLink on the GPU box, gloo in the CPU tests."""
@@ -309,6 +398,7 @@ def fit_cluster(
     distance_mode: int = 2,
     reuse_context: bool = True,
     gram_engine: int = 1,
+    devices: Optional[Sequence[int]] = None,
 ):
     """
     Cevikalp et al. 2019 convex-hull binning specialised for metagenomic binning, on B200.
@@ -324,6 +414,10 @@ def fit_cluster(
     :param num_neighbors: Number of neighbors to consider for polytope.
     :param max_iterations: Number of maximum iterations to perform.
     :param metric: Polytope distance metric (convex/affine/affine-qp).
+    :param devices: CUDA ordinals of this process to run the stage on (None: `device`, today's single-GPU path).  With two
+        or more entries and a stage large enough to pay for the exchange (sharding_pays), the query slots are sharded over
+        them as a device group (one context per entry; an ordinal may repeat) that merges the labels on the devices,
+        without torch.distributed; a smaller stage runs whole on devices[0].  Same labels and RNG draws either way.
     :return: Final binning result (int64, n).
     """
     if qp_solver != B200_SOLVER:
@@ -332,6 +426,16 @@ def fit_cluster(
         raise NotImplementedError(f"Metric {metric} not implemented")  # hull_distance.py:108
 
     dist_mod, rank, world = _dist_state()
+    if devices is not None:
+        devices = [int(dv) for dv in devices]
+        if not devices:
+            raise ValueError("devices must name at least one CUDA device")
+        if world > 1:
+            raise ValueError(f"devices={devices} shards the stage inside this process, but torch.distributed already runs it "
+                             f"on {world} ranks: use one of the two")
+        if device is not None:
+            raise ValueError("pass either device or devices")
+        device = devices[0]
     if device is None:
         device = 0
         if world > 1:
@@ -355,10 +459,16 @@ def fit_cluster(
             marks.append((label, time.perf_counter()))
 
     mark("start")
-    ctx = _get_context(device, reuse_context)
+    ctxs = [_get_context(dv, reuse_context, i) for i, dv in enumerate(devices or [device])]  # every ordinal is checked
+    ctx = ctxs[0]
+    group = None
     try:
-        ctx.set_stream(capi.OWN_STREAM)
-        ctx.reset_timers()
+        if len(ctxs) > 1 and sharding_pays(num_points_to_assign, num_clusters, len(ctxs)):
+            group = _get_group(devices, ctxs, reuse_context)
+        members = group.members if group is not None else [ctx]
+        for m in members:
+            m.set_stream(capi.OWN_STREAM)
+            m.reset_timers()
         engine = comm = None
         u0, u1 = owned_slots(num_points_to_assign, rank, world)
         if world > 1:
@@ -389,11 +499,16 @@ def fit_cluster(
             mark("features set")
         else:
             ctx.set_features(samples, asynchronous=True)  # the upload overlaps the label set-up and the first permutation draw
-        ctx.set_labels(curr, int(num_clusters), u0, u1)
-        ctx.set_params(int(num_neighbors), metric)
-        ctx.set_window(int(window))
-        ctx.set_distance_mode(int(distance_mode))
-        ctx.set_gram_engine(int(gram_engine))
+            if group is not None:
+                group.replicate_features(0)  # device to device, as the NCCL broadcast does between ranks
+        for i, m in enumerate(members):
+            if group is not None:
+                u0, u1 = owned_slots(num_points_to_assign, i, len(members))
+            m.set_labels(curr, int(num_clusters), u0, u1)
+            m.set_params(int(num_neighbors), metric)
+            m.set_window(int(window))
+            m.set_distance_mode(int(distance_mode))
+            m.set_gram_engine(int(gram_engine))
         spec_perm = spec_state = None  # a permutation drawn ahead of the iteration that will use it
         # the permutation stays on the device when the library's fused path serves the stage (chb_get_distance_path)
         on_device = world > 1 and dist_mod.get_backend() == "nccl" and ctx.distance_path() == 2
@@ -404,9 +519,15 @@ def fit_cluster(
             else:
                 spec_perm = _draw_permutation(points_to_assign, dist_mod, device)
         mark("labels/params set")
-        ctx.build_distance_matrix(bool(in_mem_dist_matrix))
+        for m in members:
+            m.build_distance_matrix(bool(in_mem_dist_matrix))
         ctx._pending_features = None
         mark("distance structure")
+        if group is not None:
+            engine = GroupEngine(group, num_points_to_assign)
+            if num_points_to_assign > 0 and max_iterations > 0:
+                exchange_guess(engine, engine, num_points_to_assign, mark)  # the group's MAX serves as the collective
+                mark("guess exchanged")
         if world > 1 and num_points_to_assign > 0 and max_iterations > 0:
             exchange_guess(engine, comm, num_points_to_assign, mark)
             mark("guess exchanged")
@@ -418,7 +539,7 @@ def fit_cluster(
         # back, so that exactly one draw per EXECUTED iteration remains visible: the reference's RNG contract.
         import contextlib
 
-        eng = engine if world > 1 else _ContextEngine(ctx)
+        eng = engine if engine is not None else _ContextEngine(ctx)
         stream_ctx = engine.stream_context() if world > 1 else contextlib.nullcontext()
         with stream_ctx:
             if spec_perm is None and max_iterations > 0:
@@ -475,15 +596,23 @@ def fit_cluster(
                            "optimal); the reference would have fallen back to cvxopt there.", tm_end["qp_iter_cap"])
         info = dict(iterations=iterations, converged=converged, changed=changed, timers=tm_end, rank=job_rank,
                     world=job_world, owned_slots=(u0, u1), replicated=job_world > 1 and world == 1)
+        if devices is not None:
+            # the device group: member i owns owned_slots(U, i, len(devices)); a stage too small to shard ran whole on devices[0]
+            info.update(world=len(devices), devices=devices, sharded=group is not None,
+                        owned_slots=[owned_slots(num_points_to_assign, i, len(members)) for i in range(len(members))])
         if marks is not None:
             info["marks_ms"] = [(lab, (t - marks[0][1]) * 1e3) for lab, t in marks]
     except BaseException:
-        _CTX_CACHE.pop(device, None)  # never reuse a context after a failure
-        ctx.close()
+        if group is not None:
+            group.close()
+        _drop(ctxs)  # never reuse a context (or a group holding it) after a failure
         raise
     finally:
         if not reuse_context:
-            ctx.close()
+            if group is not None:
+                group.close()
+            for c in ctxs:
+                c.close()
     if return_info:
         return labels, info
     return labels
@@ -501,9 +630,11 @@ def perform_clustering(
     metric: str = "convex",
     qp_solver: str = B200_SOLVER,
     in_mem_dist_matrix: bool = True,
+    devices: Optional[Sequence[int]] = None,
 ) -> Path:
     """cli/clustering.py:19-99 with steps 02-03 on the GPU.  Step 05 (FASTA dump, needs Biopython) is the
-    reference's own `dump_bins` and is only invoked when this function is installed into the reference."""
+    reference's own `dump_bins` and is only invoked when this function is installed into the reference.
+    devices: as for fit_cluster (None: one GPU; several: one stage sharded over them from this process)."""
     import pandas as pd
 
     operating_dir = Path(operating_dir)
@@ -546,9 +677,11 @@ def perform_clustering(
             distance_cache.create_distance_matrix(samples, operating_dir)
 
     logger.info(">> Performing binning using %s solver...", qp_solver)
+    multi = {} if devices is None else dict(devices=devices)  # the default call is exactly the single-GPU one
     convex_labels = fit_cluster(
         samples=samples, num_clusters=num_clusters, initial_bins=initial_bins, num_neighbors=num_neighbors,
         max_iterations=max_iterations, metric=metric, qp_solver=qp_solver, in_mem_dist_matrix=in_mem_dist_matrix,
+        **multi,
     )
     if np.any(convex_labels < 0):
         raise ValueError("There were some un-clustered points left... Aborting.")  # cli/clustering.py:79-80
@@ -563,12 +696,13 @@ def perform_clustering(
     return dist_bin_csv
 
 
-def install(ref_cli_clustering_module) -> None:
+def install(ref_cli_clustering_module, devices: Optional[Sequence[int]] = None) -> None:
     """Adds the `AlgoQpSolver = b200` branch to the reference's own `ch_bin.cli.clustering` module, in place:
     `perform_clustering(..., qp_solver="b200")` then runs steps 01-04 here (distance structure + fit_cluster on
     the GPU) and hands step 05 (FASTA dump) back to the reference's `dump_bins`; any other solver value goes
     to the untouched original.  `run_perform_clustering` (cli/clustering.py:102-127) needs no change: it looks
-    `perform_clustering` up in the module at call time."""
+    `perform_clustering` up in the module at call time.  devices: the CUDA ordinals every b200 stage runs on (None: one
+    GPU), so that the reference's single-process CLI can use several GPUs (fit_cluster's `devices`)."""
     mod = ref_cli_clustering_module
     orig_perform = mod.perform_clustering
 
@@ -579,8 +713,9 @@ def install(ref_cli_clustering_module) -> None:
                                 qp_solver, in_mem_dist_matrix)
         import pandas as pd
 
+        multi = {} if devices is None else dict(devices=devices)
         csv = perform_clustering(contig_fasta, features_csv, operating_dir, num_neighbors, max_iterations, metric,
-                                 qp_solver, in_mem_dist_matrix)
+                                 qp_solver, in_mem_dist_matrix, **multi)
         bin_dump_dir = Path(operating_dir) / "bins"
         bin_dump_dir.mkdir(parents=True, exist_ok=True)
         logger.info(">> Writing binned FASTA files...")

@@ -7,8 +7,9 @@
  * buffer it passes; no pointer is retained after the call returns (except the stream handle).
  * All functions return CHB_OK (0) or a CHB_E* code; chb_last_error() gives the message.
  * One context = one CUDA device = one host thread at a time (the reference is single-threaded,
- * ch_bin/core/clustering/algorithm.py:43-60).  Multi-GPU = one process and one context per GPU; the label
- * exchange between ranks happens above this ABI (torch.distributed / NCCL on the *_dev buffers).
+ * ch_bin/core/clustering/algorithm.py:43-60).  Multi-GPU = one context per GPU, either one process per GPU with the label
+ * exchange above this ABI (torch.distributed / NCCL on the *_dev buffers), or one process driving a device group of
+ * contexts that exchanges the labels itself (chb_group_*, below).
  *
  * There is no CPU fallback: chb_create fails with CHB_ENODEV when no sm_100 device is usable.
  */
@@ -81,7 +82,7 @@ int chb_abi_version(void);
  * AlgoQpSolver=b200 branch added at cli/clustering.py:56. */
 int chb_create(chb_ctx **out, int device_id);
 int chb_destroy(chb_ctx *ctx);
-const char *chb_last_error(const chb_ctx *ctx); /* ctx may be NULL: error of the last failed chb_create */
+const char *chb_last_error(const chb_ctx *ctx); /* ctx may be NULL: error of the last failed chb_create or chb_group_* call */
 /* Run every kernel on this cudaStream_t (e.g. a torch stream; NULL = the legacy default stream) instead of the
  * context's own non-blocking stream; pass CHB_OWN_STREAM to go back.  Needed whenever another library (NCCL via
  * torch.distributed) touches the *_dev buffers: both must be ordered on the same stream. */
@@ -262,6 +263,30 @@ int64_t chb_get_window(chb_ctx *ctx);
  * no queries) -- skip the collective and the import.  Without this pair every context computes all U guesses itself. */
 int chb_guess_export(chb_ctx *ctx, int32_t *guess_dev, int32_t *active);
 int chb_guess_import(chb_ctx *ctx, const int32_t *guess_dev);
+
+/* ---- device groups: one host thread, N contexts ------------------------------------------------------------- */
+/* A group is made of N existing, distinct contexts (one per GPU; the same device may appear more than once, each with a
+ * context of its own).  Every member keeps its own stream and owned slot range (chb_set_labels); the group only moves
+ * labels and features between members, with cudaMemcpyPeerAsync ordered by events on the members' streams.  All calls are
+ * enqueued from one host thread; errors are reported by chb_last_error(NULL).  Destroy the group before its members.
+ * The round protocol of a sharded stage over a group:
+ *   chb_group_replicate_features(g, 0)          after a chb_set_features* call on member 0, before chb_set_labels
+ *   repeat: chb_round_run(member m, lo, hi, buffer of m)   for every m
+ *           chb_group_all_max(g, hi - lo)
+ *           chb_round_commit(member m, lo, hi, buffer of m, ...)   for every m (they agree) */
+typedef struct chb_group chb_group;
+int chb_group_create(chb_group **out, chb_ctx *const *members, int32_t n);
+int chb_group_destroy(chb_group *g);
+/* A group-owned int32 device buffer of >= count entries on member m (tentative labels, guesses), on m's device.  Valid
+ * until the group is destroyed or a later call for m asks for more entries (that call waits for every member's stream). */
+int chb_group_buffer(chb_group *g, int32_t m, int64_t count, int32_t **buf_dev);
+/* Element-wise MAX over the members' group buffers [0, count), result in every member's buffer; enqueued on the members'
+ * streams, ordered after the work already enqueued there and before anything enqueued after.  Every member must hold a
+ * buffer of >= count entries. */
+int chb_group_all_max(chb_group *g, int64_t count);
+/* The feature matrix of member `root` (after any chb_set_features* call) into every other member, then what
+ * chb_features_commit derives there (asynchronously, as chb_features_commit(ctx, 1)). */
+int chb_group_replicate_features(chb_group *g, int32_t root);
 
 /* ---- measurement aid (bench.py only) ------------------------------------------------------------------ */
 /* DFMA-saturating microbenchmark: measured FP64 pipe peak of this device in TFLOP/s (FMA = 2 flop). */
