@@ -3,14 +3,19 @@ GPU parity tests proper: every check goes through the C-ABI (chbin_b200.capi.Con
 compared with the CPU oracle (oracle/*.c) on the same seeded inputs.  Bars: bit-exact for distances, kNN index
 sets and labels; |d_gpu - d_ref| <= 1e-6*d_ref + 1e-12*||x|| for hull distances (BASELINE.md section 4).
 """
+import os
+
 import numpy as np
 import pytest
 
 import chbin_b200
+import fused_invariants
 import oracle
 from chbin_b200 import capi, synth
 
 pytestmark = pytest.mark.gpu
+
+THREADS = os.cpu_count() or 1
 
 
 def _ctx(X, bins, C, k, metric="convex", materialise=True, slots=(0, -1), dist_mode=1, gram_engine=1):
@@ -220,11 +225,11 @@ def test_fit_cluster_fused_with_duplicate_contigs():
 def test_fused_keys_within_proven_bound_and_lists_complete(n, C, S, k):
     """Distance mode 2 (fused.cu): every FP32 key the fused Gram + selection kernel kept must lie within the per-(query,
     bin) slack of the exact squared distance (per-bin centred operands), and the kept lists must contain every point
-    whose exact distance is among the k smallest of its bin -- the two facts the exact re-rank relies on."""
+    whose exact distance is among the k smallest of its bin -- the two facts the exact re-rank relies on.  Also the rest
+    of tests/fused_invariants.py: cached sets and hull distances, pruning, row bounds, guess."""
     X, bins, _ = synth.make_contig_features(n, C, S, 12, seed=29)
     perms = oracle.draw_permutations(bins, 2, seed=0)
-    D = oracle.create_in_mem_distance_matrix(X)
-    pts = np.where(bins == -1)[0]
+    ref = fused_invariants.Reference(X, bins, C, k)
     ctx = capi.Context(0)
     ctx.set_features(X); ctx.set_params(k, "convex"); ctx.set_distance_mode(2); ctx.set_labels(bins, C)
     ctx.build_distance_matrix(True)
@@ -232,33 +237,7 @@ def test_fused_keys_within_proven_bound_and_lists_complete(n, C, S, k):
     worst = 0.0
     for it in range(2):
         lab, _ = ctx.fit_iteration(perms[it])
-        key, idx, slack = ctx.get_fused_candidates(0, len(pts))
-        _, pcnt, pdist = ctx.get_pair_cache(0, len(pts))
-        pruned = (pcnt == 0) & np.isinf(pdist)  # bins ruled out by the bounds (or empty): lists not maintained
-        pos = np.full(len(X), -1)
-        pos[perms[it]] = np.arange(len(perms[it]))
-        for u, j in enumerate(pts):
-            for c in range(C):
-                if pruned[u, c]:
-                    continue
-                valid = np.isfinite(key[u, c])
-                ii = idx[u, c][valid]
-                d2 = D[j, ii] ** 2
-                err = np.abs(key[u, c][valid].astype(np.float64) - d2)
-                assert np.all(err <= slack[u, c]), (it, j, c, err.max(), slack[u, c])
-                if len(err):
-                    worst = max(worst, float((err / slack[u, c]).max()))
-            if u % 5 == 0:  # the last round's lists were formed on the final labels as seen from this query's position
-                eff = np.where(pos < pos[j], lab, cur)
-                eff[j] = -1
-                hd = [oracle.convex_hull_distance(X[j], X[oracle.find_nearest_from_cluster(c, eff, D[j], k)])
-                      if np.any(eff == c) else np.inf for c in range(C)]
-                for c in range(C):
-                    want = oracle.find_nearest_from_cluster(c, eff, D[j], k)
-                    if pruned[u, c]:
-                        assert len(want) == 0 or hd[c] > min(hd), (it, j, c)  # a pruned bin is never the nearest hull
-                    else:
-                        assert set(want.tolist()) <= set(idx[u, c][np.isfinite(key[u, c])].tolist()), (it, j, c)
+        worst = max(worst, fused_invariants.check_iteration(ctx, ref, perms[it], cur, lab, threads=THREADS)["worst"])
         cur = lab
     ctx.close()
     assert worst < 0.5, f"observed error / bound = {worst}: the bound should have a wide margin"

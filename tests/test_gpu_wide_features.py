@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 import chbin_b200
+import fused_invariants
 import oracle
 from chbin_b200 import capi, synth
 
@@ -95,56 +96,29 @@ def test_wide_fused_duplicates_tiny_bins_and_bins_without_seeds(wide_fused, d, k
 @pytest.mark.parametrize("d,k", [(528, 5), (1024, 10)])
 def test_wide_fused_keys_within_proven_bound_and_lists_complete(wide_fused, d, k):
     """The kept FP32 keys of the streamed kernel lie within the per-(query, bin) slack of the exact squared distance, the
-    kept lists hold every true neighbour, and a pruned bin is never the nearest hull."""
+    kept lists hold every true neighbour, and a pruned bin is never the nearest hull (tests/fused_invariants.py)."""
     C = 5
     X, bins, _ = _features(1300, C, d, 12, seed=29 + d)
     perms = oracle.draw_permutations(bins, 2, seed=0)
-    D = oracle.create_in_mem_distance_matrix(X)
-    pts = np.where(bins == -1)[0]
+    ref = fused_invariants.Reference(X, bins, C, k)
     ctx = capi.Context(0)
     ctx.set_features(X); ctx.set_params(k, "convex"); ctx.set_distance_mode(2); ctx.set_labels(bins, C)
     assert ctx.distance_path() == 2
     ctx.build_distance_matrix(True)
     cur = bins.copy()
-    worst, checked = 0.0, 0
+    worst = 0.0
     for it in range(2):
         lab, _ = ctx.fit_iteration(perms[it])
-        key, idx, slack = ctx.get_fused_candidates(0, len(pts))
-        _, pcnt, pdist = ctx.get_pair_cache(0, len(pts))
-        pruned = (pcnt == 0) & np.isinf(pdist)
-        pos = np.full(len(X), -1)
-        pos[perms[it]] = np.arange(len(perms[it]))
-        for u, j in enumerate(pts):
-            for c in range(C):
-                if pruned[u, c]:
-                    continue
-                valid = np.isfinite(key[u, c])
-                d2 = D[j, idx[u, c][valid]] ** 2
-                err = np.abs(key[u, c][valid].astype(np.float64) - d2)
-                assert np.all(err <= slack[u, c]), (it, j, c, err.max(), slack[u, c])
-                if len(err):
-                    worst = max(worst, float((err / slack[u, c]).max()))
-                    checked += len(err)
-            if u % 4 == 0:
-                eff = np.where(pos < pos[j], lab, cur)
-                eff[j] = -1
-                want = [oracle.find_nearest_from_cluster(c, eff, D[j], k) for c in range(C)]
-                hd = [oracle.convex_hull_distance(X[j], X[w]) if len(w) else np.inf for w in want]
-                for c in range(C):
-                    if pruned[u, c]:
-                        assert len(want[c]) == 0 or hd[c] > min(hd), (it, j, c)
-                    else:
-                        assert set(want[c].tolist()) <= set(idx[u, c][np.isfinite(key[u, c])].tolist()), (it, j, c)
+        worst = max(worst, fused_invariants.check_iteration(ctx, ref, perms[it], cur, lab, threads=THREADS)["worst"])
         cur = lab
     ctx.close()
-    assert checked > 0
     assert worst < 0.5, f"observed error / bound = {worst}: the bound should have a wide margin"
 
 
 def test_wide_row_bounds_hold_on_large_cancelling_coordinates(wide_fused):
     """d = 1024, features far from the global mean (|x - mu| ~ 1e3) with in-bin offsets ~1e-2: the FP32 differences cancel
     almost completely.  For every row the pruning bounds must still hold against exact FP64 distances to the seeds of the
-    guessed bin: ub >= the nearest one, ubk2 >= the k-th smallest squared one."""
+    guessed bin: ub >= the nearest one, ubk2 >= the k-th smallest squared one (with the rest of tests/fused_invariants.py)."""
     rng = np.random.default_rng(5)
     n, d, C, k, n_seed = 1200, 1024, 4, 5, 40
     truth = np.arange(n) % C
@@ -154,21 +128,16 @@ def test_wide_row_bounds_hold_on_large_cancelling_coordinates(wide_fused):
     bins = np.full(n, -1, dtype=np.int64)
     for c in range(C):
         bins[np.where(truth == c)[0][:n_seed]] = c
-    pts = np.where(bins == -1)[0]
+    ref = fused_invariants.Reference(X, bins, C, k)
+    perm = oracle.draw_permutations(bins, 1, seed=0)[0]
     ctx = capi.Context(0)
     ctx.set_features(X); ctx.set_params(k, "convex"); ctx.set_distance_mode(2); ctx.set_labels(bins, C)
     ctx.build_distance_matrix(True)
-    ctx.fit_iteration(oracle.draw_permutations(bins, 1, seed=0)[0])
-    guess, ub, ubk2 = ctx.get_row_bounds(0, len(pts))
+    lab, _ = ctx.fit_iteration(perm)
+    guess, _, _ = ctx.get_row_bounds(0, len(ref.pts))
+    fused_invariants.check_iteration(ctx, ref, perm, bins, lab, threads=THREADS)
     ctx.close()
     assert np.all(guess < C)
-    for u, j in enumerate(pts):
-        seeds = np.where(bins == guess[u])[0]
-        dist = np.sqrt(np.sum((X[seeds] - X[j]) ** 2, axis=1))
-        assert float(ub[u]) >= dist.min(), (j, float(ub[u]), dist.min())
-        kth2 = np.sort(dist ** 2)[k - 1]
-        assert float(ubk2[u]) >= kth2, (j, float(ubk2[u]), kth2)
-        assert float(ub[u]) <= dist.min() * (1 + 1e-3) + 1e-3, "the bound should be tight"
 
 
 @pytest.mark.parametrize("on_device", [False, True])
